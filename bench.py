@@ -2,7 +2,7 @@
 """Benchmark of the ChronoEdit denoising hot path (BASELINE.json metric: DiT denoising steps/sec at 14B, 720x1280,
 5 pixel frames = 2 latent frames).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" = one iteration of the sampling loop of ChronoEditPipeline.__call__ (pipeline_chronoedit.py:695-753) for ONE
 edit with classifier-free guidance: two DiT forwards (prompt / negative prompt — evaluated as one batch-2 call, which the
@@ -20,6 +20,10 @@ Printed JSON (one line, rank 0):
             with CUDA events inside the timed region, against MEASURED_PEAKS.json bf16_tflops_sustained
   cpu_baseline  the oracle (CPU restatement of the reference) timed on the host cores on a bounded sample
 --impl reference times that CPU path alone with the same metric/config (the reference has no faster path on this box).
+
+--dump-outputs DIR writes what the last timed step computed on rank 0 as float32 .npy files: noise_pred.npy (the batch-2 DiT
+output, conditional then unconditional) and latents.npy (the latents the guided scheduler step returned).  Weights and inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -350,6 +354,8 @@ def run_ours(args):
     d_lat = d_lat.to(torch.bfloat16)   # the diffusers pipeline keeps bf16 latents (pipeline_chronoedit.py:676-687)
     d_in = torch.cat([d_lat, d_cond], dim=1).contiguous()
 
+    last = {}
+
     def device_step(i):
         nonlocal d_lat
         if sched.step_index is None or sched.step_index >= 50:
@@ -357,6 +363,8 @@ def run_ours(args):
         t = sched.timesteps[sched.step_index or 0]
         out = model(d_in.expand(2, -1, -1, -1, -1), t.expand(2), d_text, d_img, return_dict=False)[0]
         d_lat = sched.step_cfg(out[0:1], out[1:2], GUIDANCE, t, d_lat, model_input_out=d_in)
+        if args.dump_outputs:
+            last["noise_pred"], last["latents"] = out, d_lat
 
     # host-buffer (e2e) step = the SAME loop body through the host-facing call: every step the model input (built on the host from
     # the host copy of the latents), the timestep and the prompt / image embeddings go pinned-host -> device inside
@@ -440,6 +448,12 @@ def run_ours(args):
             device_step(args.warmup + i)
         model.clear_context_cache()
     dev_ms, wall_ms, _, clocks = timed(counted_step, args.steps, 0, sampler, profile=False)
+    if args.dump_outputs and rank == 0:   # before the passes below overwrite the model's output buffer and the latents
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, v in last.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), v.float().cpu().numpy())
     model.use_cuda_graph = False
     launches = launch_count["n"]
     value = world * args.steps / (dev_ms / 1000.0)
@@ -598,7 +612,10 @@ def main():
     ap.add_argument("--no-vae", action="store_true", help="skip the (untimed-region) VAE encode/decode measurement")
     ap.add_argument("--latent-frames", type=int, default=2, choices=[2, 8],
                     help="DEV ONLY: 8 = the temporal-reasoning geometry of configs[2] (28 800 tokens); not the headline workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's DiT output and new latents to DIR/*.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path; --impl reference has none")
     if args.latent_frames != 2:
         global FRAMES
         FRAMES = args.latent_frames

@@ -45,6 +45,9 @@ PIPELINE_CASES: Dict[str, PipelineCase] = {
 
 DIT_CFG = D.DiTConfig.tiny()
 VAE_CFG = V.VAEConfig.tiny(32)
+# torch's bf16 matrix products on the CPU (oneDNN) round differently with the number of intra-op threads, and the difference
+# grows over the denoising steps; the stored pipeline videos are made and compared with this many threads
+GOLDEN_THREADS = 8
 
 
 def weights():

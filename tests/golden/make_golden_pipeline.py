@@ -30,7 +30,7 @@ OUT = os.path.dirname(os.path.abspath(__file__))
 
 def main():
     assert ref_loader.reference_available(), "run this in the build container (needs /root/reference)"
-    torch.set_num_threads(os.cpu_count() or 1)
+    torch.set_num_threads(pipeline_cases.GOLDEN_THREADS)
     manifest = {"torch": torch.__version__, "generated_by": "tests/golden/make_golden_pipeline.py", "cases": {}}
     for name, case in pipeline_cases.PIPELINE_CASES.items():
         ref16 = pipeline_cases.run_reference_pipeline(case, torch.bfloat16)

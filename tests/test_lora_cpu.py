@@ -1,12 +1,14 @@
 """CPU tests (-m "not gpu") of `ChronoEditTransformer3DModel.fuse_lora`: the merge arithmetic (W += (B @ A) * s * alpha / r in
 the weight dtype), the two key conventions (diffusers / PEFT names and the original Wan names the in-tree loader handles,
-chronoedit/_src/models/utils.py:66-190), and the Wan <-> diffusers module map against the reference's own state-dict
-converter (chronoedit_diffsynth/wan_video_dit_chronoedit.py:434-541) when /root/reference is present."""
+chronoedit/_src/models/utils.py:66-190), and the Wan <-> diffusers module map against what the reference's own state-dict
+converter (chronoedit_diffsynth/wan_video_dit_chronoedit.py:434-541) made of the same names (tests/golden/make_golden_lora.py)."""
+import json
+import os
+
 import pytest
 import torch
 
 from oracle import dit_oracle as O
-from oracle import ref_loader
 
 
 def _model():
@@ -135,19 +137,14 @@ def test_diffusers_style_load_then_fuse():
         m2.fuse_lora(0.75)   # already merged: nothing left to fuse, and certainly not twice
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="/root/reference only exists in the build container")
-def test_wan_to_diffusers_module_map_matches_reference_converter():
+def test_wan_to_diffusers_module_map_matches_reference_converter(golden_dir):
     import chronoedit_b200 as ce
-    ds = ref_loader.load_reference_diffsynth_dit()
-    src = open(ds.__file__).read()
+    with open(os.path.join(golden_dir, "LORA_MANIFEST.json")) as f:
+        to_wan = json.load(f)["converter_wan_key_of_diffusers_key"]
     for wan, dif in ce.ChronoEditTransformer3DModel._WAN_TO_DIFFUSERS:
-        if "k_img" in wan or "v_img" in wan:
-            continue   # image k/v projections: checked below against whichever spelling the converter uses
-        assert f'"blocks.0.{dif}.weight": "blocks.0.{wan}.weight"' in src, (wan, dif)
-    assert '"blocks.0.attn2.add_k_proj.weight": "blocks.0.cross_attn.k_img.weight"' in src
-    assert '"blocks.0.attn2.add_v_proj.weight": "blocks.0.cross_attn.v_img.weight"' in src
+        assert to_wan[f"blocks.0.{dif}.weight"] == f"blocks.0.{wan}.weight", (wan, dif)
     for wan, dif in ce.ChronoEditTransformer3DModel._WAN_TO_DIFFUSERS_GLOBAL.items():
-        assert f'"{dif}.weight": "{wan}.weight"' in src, (wan, dif)
+        assert to_wan[f"{dif}.weight"] == f"{wan}.weight", (wan, dif)
 
 
 def test_new_weights_drop_the_context_cache():

@@ -1,35 +1,42 @@
 """Pipeline-level boundary tests that run WITHOUT a GPU (-m "not gpu").
 
-(1) Pin of oracle/pipeline_oracle.py: the UNMODIFIED reference pipeline file
-    (/root/reference/chronoedit_diffusers/pipeline_chronoedit.py, `ChronoEditPipeline.__call__` :484-812) is executed through
-    oracle/diffusers_shim with the reference's own transformer / VAE twin / flow-UniPC scheduler, and the restatement driven by the
-    oracle modules must reproduce its video bit for bit -- with and without the temporal-reasoning cut (:700-709) and the
-    two-decode tail (:776-779).  Build container only (needs /root/reference); everywhere else the restatement is held against
-    the stored reference outputs (tests/golden/pipeline_*.safetensors).
-(2) Drop-in surface: the same UNMODIFIED pipeline is run with the three chronoedit_b200 mirrors registered in place of the
-    reference's objects.  There is no GPU here and the mirrors have no CPU path, so their three native seams (`_native_forward`,
+(1) Pin of oracle/pipeline_oracle.py: the UNMODIFIED reference pipeline (chronoedit_diffusers/pipeline_chronoedit.py,
+    `ChronoEditPipeline.__call__` :484-812), executed through oracle/diffusers_shim with the reference's own transformer / VAE
+    twin / flow-UniPC scheduler, produced the videos stored in tests/golden/pipeline_*.safetensors
+    (tests/golden/make_golden_pipeline.py); the restatement driven by the oracle modules must reproduce them bit for bit --
+    with and without the temporal-reasoning cut (:700-709) and the two-decode tail (:776-779).
+(2) Drop-in surface: the pipeline loop pinned in (1) is run with the three chronoedit_b200 mirrors in place of the oracle's
+    objects.  There is no GPU here and the mirrors have no CPU path, so their three native seams (`_native_forward`,
     `_native_encode/_native_decode`, `_native_step`) are stood in for by the oracle -- everything else (constructor surface,
     `.config`, `.dtype`, `temperal_downsample`, argument handling, return types, the scheduler state the pipeline slices in
     place, LoRA loading through `pipe.load_lora_weights / fuse_lora`) is the product code, and the video must equal the
     reference's.  The GPU twin of this test (tests/test_gpu_pipeline.py) runs the real kernels under the same loop.
 """
+import hashlib
+import json
 import os
 
 import pytest
 import torch
 from safetensors.torch import load_file
 
-from oracle import cases, dit_oracle as D, pipeline_cases as PC, pipeline_oracle as P, ref_loader, unipc_oracle as U, vae_oracle as V
+from oracle import cases, dit_oracle as D, pipeline_cases as PC, pipeline_oracle as P, unipc_oracle as U, vae_oracle as V
 
-needs_ref = pytest.mark.skipif(not ref_loader.reference_available(), reason="/root/reference only exists in the build container")
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
-@needs_ref
+@pytest.fixture(autouse=True)
+def _golden_thread_count():
+    n = torch.get_num_threads()
+    torch.set_num_threads(PC.GOLDEN_THREADS)
+    yield
+    torch.set_num_threads(n)
+
+
 @pytest.mark.parametrize("name", list(PC.PIPELINE_CASES))
 def test_pipeline_restatement_is_bit_identical_to_the_unmodified_pipeline(name):
     case = PC.PIPELINE_CASES[name]
-    ref = PC.run_reference_pipeline(case, torch.bfloat16)
+    ref = load_file(os.path.join(GOLDEN, f"pipeline_{name}.safetensors"))["video_ref_bf16"]
     ora = PC.run_oracle_pipeline(case, torch.bfloat16)
     assert ref.shape == ora.shape and ref.dtype == ora.dtype
     assert torch.equal(ref, ora), float((ref.float() - ora.float()).abs().max())
@@ -42,12 +49,13 @@ def test_pipeline_restatement_matches_stored_reference_output(name):
     ora = PC.run_oracle_pipeline(case, torch.bfloat16).float()
     ref = gold["video_ref_bf16"].float()
     assert ora.shape == ref.shape
-    # same torch build / CPU kernels -> identical; a different CPU (other bf16 GEMM paths) may flip isolated bf16 ulps
+    # same torch build / CPU kernels / thread count -> identical; a different CPU (other bf16 GEMM paths) may flip isolated
+    # bf16 ulps
     assert (ora - ref).abs().mean() <= 2e-3 and (ora - ref).abs().max() <= 0.1
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# (2) the unchanged pipeline with the mirrors
+# (2) the pipeline loop with the mirrors
 # ---------------------------------------------------------------------------------------------------------------------
 def _mirror_transformer(dsd):
     import chronoedit_b200 as ce
@@ -104,24 +112,19 @@ def _mirror_scheduler(shift):
     return s
 
 
-@needs_ref
 @pytest.mark.parametrize("name", list(PC.PIPELINE_CASES))
-def test_unmodified_pipeline_drives_the_mirrors(name):
+def test_pipeline_drives_the_mirrors(name):
     case = PC.PIPELINE_CASES[name]
     dsd, vsd = PC.weights()
-    ref = PC.run_reference_pipeline(case, torch.bfloat16)
+    ref = load_file(os.path.join(GOLDEN, f"pipeline_{name}.safetensors"))["video_ref_bf16"]
     tr, vae, sch = _mirror_transformer(dsd), _mirror_vae(vsd), _mirror_scheduler(case.sched_shift)
-    got = PC.run_reference_pipeline(case, torch.bfloat16, transformer=tr, vae=vae, scheduler=sch)
+    got = PC.run_oracle_pipeline(case, torch.bfloat16, transformer=tr, vae=vae, scheduler=sch)
     assert got.shape == ref.shape
     assert torch.equal(got, ref), float((got.float() - ref.float()).abs().max())
 
 
-@needs_ref
-def test_cli_lora_lines_work_on_the_mirror():
-    """run_inference_diffusers.py:369-376: pipe.load_lora_weights(path); pipe.fuse_lora(lora_scale=s) -- through the pipeline's
-    WanLoraLoaderMixin into the transformer mirror; the video must equal the reference modules run on the merged weights."""
-    case = PC.PIPELINE_CASES["edit_nocfg"]
-    dsd, vsd = PC.weights()
+def _cli_lora(dsd):
+    """A seeded LoRA file in diffusers / PEFT key style over six of the projections of every block."""
     g = torch.Generator().manual_seed(5)
     lora = {}
     for k, w in dsd.items():
@@ -129,16 +132,38 @@ def test_cli_lora_lines_work_on_the_mirror():
             mod = k[: -len(".weight")]
             lora[f"transformer.{mod}.lora_A.weight"] = (torch.randn(4, w.shape[1], generator=g) * 0.2).bfloat16()
             lora[f"transformer.{mod}.lora_B.weight"] = (torch.randn(w.shape[0], 4, generator=g) * 0.2).bfloat16()
+    return lora
+
+
+def _video_sha256(video):
+    return hashlib.sha256(video.contiguous().view(torch.int16).numpy().tobytes()).hexdigest()
+
+
+def test_cli_lora_lines_work_on_the_mirror():
+    """run_inference_diffusers.py:369-376: pipe.load_lora_weights(path); pipe.fuse_lora(lora_scale=s) -- through the
+    WanLoraLoaderMixin that ChronoEditPipeline takes both from, into the transformer mirror; the video must equal the oracle
+    modules run on the merged weights, and the video the unmodified pipeline made from the same mirror (recorded as a digest
+    by tests/golden/make_golden_lora.py)."""
+    from oracle.diffusers_shim.diffusers.loaders import WanLoraLoaderMixin
+
+    class Pipe(WanLoraLoaderMixin):
+        def __init__(self, transformer):
+            self.transformer = transformer
+
+    case = PC.PIPELINE_CASES["edit_nocfg"]
+    dsd, vsd = PC.weights()
+    lora = _cli_lora(dsd)
     tr = _mirror_transformer(dsd)
-    pl = ref_loader.load_reference_pipeline()
-    pipe = pl.ChronoEditPipeline(tokenizer=None, text_encoder=None, image_encoder=None, image_processor=None, transformer=tr,
-                                 vae=_mirror_vae(vsd), scheduler=_mirror_scheduler(case.sched_shift), disable_guardrails=True)
+    pipe = Pipe(tr)
     pipe.load_lora_weights(lora)
     pipe.fuse_lora(lora_scale=0.8)
     merged = {k: v.clone() for k, v in tr.state_dict().items()}
     base = cases.to_bf16_state(dsd)
     changed = [k for k in merged if not torch.equal(merged[k], base[k])]
     assert len(changed) == len(lora) // 2
-    got = PC.run_reference_pipeline(case, torch.bfloat16, transformer=tr, vae=pipe.vae, scheduler=pipe.scheduler)
+    got = PC.run_oracle_pipeline(case, torch.bfloat16, transformer=tr, vae=_mirror_vae(vsd), scheduler=_mirror_scheduler(case.sched_shift))
     want = PC.run_oracle_pipeline(case, torch.bfloat16, transformer=P.OracleTransformer(merged, PC.DIT_CFG, torch.bfloat16))
     assert torch.equal(got, want)
+    with open(os.path.join(GOLDEN, "LORA_MANIFEST.json")) as f:
+        ref = json.load(f)["cli_lora_video"]
+    assert list(got.shape) == ref["shape"] and _video_sha256(got) == ref["sha256"]

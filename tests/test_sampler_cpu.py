@@ -1,6 +1,6 @@
 """CPU tests (-m "not gpu") of the sampling-glue row: the oracle restatement of FlowUniPCMultistepScheduler reproduces the
-golden vectors recorded from the unmodified reference (and the live reference when /root/reference is present); the product
-mirror's host-side logic (sigma schedule, per-step scalars, bookkeeping, error behaviour) agrees with both."""
+golden vectors recorded from the unmodified reference (tests/golden/make_golden_unipc.py); the product mirror's host-side
+logic (sigma schedule, per-step scalars, bookkeeping, error behaviour) agrees with both."""
 import json
 import os
 
@@ -9,7 +9,7 @@ import pytest
 import torch
 from safetensors.torch import load_file
 
-from oracle import ref_loader, unipc_oracle
+from oracle import unipc_oracle
 from oracle.unipc_cases import UNIPC_CASES, case_inputs
 
 
@@ -47,18 +47,14 @@ def test_oracle_matches_golden_bit_exact(name, golden_dir):
         assert torch.equal(_bits(x), _bits(g)), f"{name}: step {i} differs from the reference"
 
 
-@pytest.mark.skipif(not ref_loader.reference_available(), reason="/root/reference only exists in the build container")
-def test_oracle_matches_live_reference():
-    ref = ref_loader.load_reference_unipc()
+def test_oracle_matches_live_reference(golden_dir):
+    """The reference scheduler stepped by the pipeline's own guidance combine (pipeline_chronoedit.py:736), as stored by
+    make_golden_unipc.py."""
     case = UNIPC_CASES["bf16_cfg_10step"]
-    sch = ref.FlowUniPCMultistepScheduler(num_train_timesteps=1000, shift=1, use_dynamic_shifting=False)
-    sch.set_timesteps(case.steps, device="cpu", shift=case.shift)
-    x, cond, uncond = case_inputs(case)
+    gold = load_file(os.path.join(golden_dir, "unipc_bf16_cfg_10step.safetensors"))
     _, outs = _run_oracle(case)
-    for i, t in enumerate(sch.timesteps):
-        v = uncond[i] + case.guidance * (cond[i] - uncond[i])
-        x = sch.step(v, t, x, return_dict=False)[0]
-        assert torch.equal(_bits(x), _bits(outs[i]))
+    for i in range(case.steps):
+        assert torch.equal(_bits(gold[f"step{i:02d}"]), _bits(outs[i]))
 
 
 def test_cuda_scalar_semantics_distance_is_as_recorded(golden_dir):
